@@ -5,6 +5,7 @@
   python bench.py --gpus 1 --steps K --warmup W                 # our engine (libsfb200 on B200)
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference --gpus N --steps K --warmup W  # the reference's CPU path (oracle port) on the host
+  python bench.py ... --dump-outputs DIR                        # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one training iteration = one rollout of 32 env steps for all envs of the rank (131 072 env steps) followed
 by one learner pass (4 minibatches x 1 epoch, forward + backward + Adam).  Prints ONE JSON line (rank 0).
@@ -160,7 +161,7 @@ def oracle_cpu_run(steps: int, warmup: int, n_envs: int = N_ENVS, calibrate: boo
 
 
 def _ref_driver_call(n_envs: int, steps: int, warmup: int, threads: int, timeout: int = 1500):
-    """One run of the UNMODIFIED reference (baseline/_ref, driven by oracle/ref_driver.py) in a subprocess (its logger is
+    """One run of the UNMODIFIED reference (oracle/_ref, driven by oracle/ref_driver.py) in a subprocess (its logger is
     chatty and its thread settings are process-wide).  Returns the result dict or None."""
     cmd = [sys.executable, "-m", "oracle.ref_driver", "--n_envs", str(n_envs), "--rollout", str(ROLLOUT), "--obs_dim",
            str(OBS_DIM), "--num_actions", str(N_ACTIONS), "--batch_size", str(n_envs * ROLLOUT // N_MINIBATCH),
@@ -178,9 +179,9 @@ def _ref_driver_call(n_envs: int, steps: int, warmup: int, threads: int, timeout
 
 
 def reference_cpu_run(steps: int, warmup: int, n_envs: int = N_ENVS):
-    """The reference's own CPU implementation of the path (sample-factory 2.1.3 installed in baseline/_ref): serial mode,
+    """The reference's own CPU implementation of the path (sample-factory 2.1.3 installed in oracle/_ref): serial mode,
     batched sampling, torch CPU.  torch CPU throughput on this workload is not monotone in the thread count, so the count
-    is calibrated on a reduced run (1024 envs) and reported as `cores`.  None when baseline/_ref is absent."""
+    is calibrated on a reduced run (1024 envs) and reported as `cores`.  None when oracle/_ref is absent."""
     from oracle import ref_driver
 
     if not ref_driver.available():
@@ -206,13 +207,13 @@ def run_reference(args):
     r = reference_cpu_run(args.steps, args.warmup, n_envs)
     if r is not None:
         kind = "reference"
-        sample = (f"{what}; the unmodified reference (sample-factory 2.1.3 pip-installed into baseline/_ref) driven through "
+        sample = (f"{what}; the unmodified reference (sample-factory 2.1.3 pip-installed into oracle/_ref) driven through "
                   f"BatchedVectorEnvRunner + ActorCritic forward + Learner.train, serial mode, torch CPU, "
                   f"{r['cores']} of {os.cpu_count()} host threads (best of a calibration sweep)")
     else:
         kind = "port"
         r = oracle_cpu_run(args.steps, args.warmup, n_envs)
-        sample = (f"{what}; oracle port (baseline/_ref absent), torch CPU with the best-performing intra-op thread count "
+        sample = (f"{what}; oracle port (oracle/_ref absent), torch CPU with the best-performing intra-op thread count "
                   f"({r['cores']} of {os.cpu_count()} host threads)")
     workload = WORKLOAD if args.gpus == 1 else WORKLOAD.replace("4096 envs per GPU", f"{n_envs} envs (= 4096 per GPU of our arm)")
     out = dict(impl="reference", metric=METRIC, value=r["value"], unit=UNIT, n_gpus=args.gpus, steps=args.steps,
@@ -332,6 +333,29 @@ def dp_check(rank: int, world: int, dev, engine_flag: str, bench_model) -> dict:
                    shape=f"{world} ranks x {n} envs x {ROLLOUT} steps vs 1 process x {n_all} envs, {n_iter} iterations, 10% invalid samples")
     dist.barrier()
     return out
+
+
+def timed_path_outputs(runner) -> dict:
+    """Host copies of what the last Runner.iteration() left for its caller: the trajectories of its rollout (what the learner
+    trained on), the learner's advantages / returns / per-minibatch loss terms / grad norms, and the trained policy's
+    state_dict (weights + normaliser statistics).  float64 stays float64, everything else becomes float32 (44 MB)."""
+    lrn = runner.learner
+    n = lrn.num_minibatches_done
+    out = {f"traj.{k}": v for k, v in runner.traj.items()}
+    out.update({"learner.advantages": lrn.advantages, "learner.returns": lrn.returns,
+                "learner.loss_stats": lrn.loss_stats_log[:n], "learner.grad_norm": lrn.grad_norm_log[:n]})
+    out.update({f"model.{k}": v for k, v in runner.model.state_dict().items()})
+    return {k: v.detach().cpu().numpy().astype("float64" if v.dtype == torch.float64 else "float32") for k, v in out.items()}
+
+
+def write_outputs(path: str, arrays: dict) -> None:
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes exceed 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def run_ours(args):
@@ -454,6 +478,7 @@ def run_ours(args):
     barrier()
     timing_on[0] = False
     ms_total = max_over_ranks(e0.elapsed_time(e1))
+    outputs = timed_path_outputs(runner) if (args.dump_outputs and rank == 0) else None
     gpu_launches = (ops.launch_count() - launches0) + replay_launches
     learner_graphed = bool(runner.learner.use_graph)
     if runner.learner.use_graph:
@@ -641,7 +666,7 @@ def run_ours(args):
         if r is not None:
             cpu_baseline = dict(value=r["value"], unit=UNIT, cores=r["cores"], kind="reference", ms_per_step=r["ms_per_step"],
                                 sample="6 full iterations (4096 envs x 32 steps + learner) after 2 warm-up; the unmodified reference "
-                                       "(sample-factory 2.1.3 in baseline/_ref: BatchedVectorEnvRunner + ActorCritic + Learner.train, "
+                                       "(sample-factory 2.1.3 in oracle/_ref: BatchedVectorEnvRunner + ActorCritic + Learner.train, "
                                        f"serial mode, torch CPU), {r['cores']} of {os.cpu_count()} host threads")
         rp = oracle_cpu_run(steps=6, warmup=2)
         port = dict(value=rp["value"], unit=UNIT, cores=rp["cores"], kind="port", ms_per_step=rp["ms_per_step"],
@@ -652,6 +677,8 @@ def run_ours(args):
         else:
             cpu_baseline["oracle_port"] = port
 
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         out = dict(metric=METRIC, value=value, unit=UNIT, n_gpus=world, steps=args.steps, warmup=args.warmup,
                    ms_per_step=ms_per_step, higher_is_better=True, scaling="weak", vs_baseline=None,
@@ -704,7 +731,14 @@ def main():
                     help="N > 1: skip the (untimed) replica / single-GPU equivalence check printed as `dp_check`")
     ap.add_argument("--no-strong", dest="no_strong", action="store_true",
                     help="N > 1: skip the strong-scaling point (4096 envs in total, split over the ranks)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (trajectories, advantages / returns, loss "
+                         "terms, trained state_dict; rank 0) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs applies to the headline workload of our engine (--impl ours --config 2)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.config != 2:
         import bench_configs

@@ -1,8 +1,8 @@
 """TEST / MEASUREMENT INFRASTRUCTURE ONLY -- never imported by the product (sample_factory_b200/).
 
-Drives the UNMODIFIED reference (alex-petrenko/sample-factory 2.1.3, pip-installed by `__graft_entry__.build()` into
-baseline/_ref with `pip install --no-index --no-deps --target baseline/_ref /root/reference`) through its own classes on
-the host CPU, for `bench.py --impl reference` and the `cpu_baseline` leg:
+Drives the UNMODIFIED reference (alex-petrenko/sample-factory 2.1.3, pip-installed into oracle/_ref by
+`__graft_entry__.build()`, oracle/build_ref.py) through its own classes on the host CPU, for `bench.py --impl reference`
+and the `cpu_baseline` leg:
 
     BatchedVectorEnvRunner.{init, update_trajectory_buffers, generate_policy_request, advance_rollouts}
                                                            (algo/sampling/batched_sampling.py:154-388)
@@ -24,11 +24,13 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF_DIR, "sample_factory", "algo", "learning", "learner.py"))
+    from oracle import build_ref
+
+    return build_ref.installed(REF_DIR)
 
 
 def run(n_envs: int, rollout: int, obs_dim: int, num_actions: int, hidden, batch_size: int, num_batches_per_epoch: int,
@@ -143,7 +145,7 @@ def run(n_envs: int, rollout: int, obs_dim: int, num_actions: int, hidden, batch
             times.append(dt)
     total = sum(times)
     return dict(value=n_envs * rollout * len(times) / total, ms_per_step=1e3 * total / len(times), cores=threads,
-                train_step=int(learner.train_step), version="sample-factory 2.1.3 (baseline/_ref)")
+                train_step=int(learner.train_step), version="sample-factory 2.1.3 (oracle/_ref)")
 
 
 def main(argv=None) -> None:

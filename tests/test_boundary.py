@@ -2,8 +2,8 @@
 model registry exists, plain gymnasium-API envs are adapted automatically, and the reference's own example script
 `sf_examples/train_gym_env.py` (BASELINE.json config 1: CartPole-v1) runs UNMODIFIED against this repository.
 
-The example scripts are reference code: they are executed from where the reference lives (baseline/_ref, the pip-installed
-reference that travels to the GPU box; /root/reference in the build container) -- never copied into the repo."""
+The example scripts are reference code: they are executed from the reference that __graft_entry__.build() pip-installs into
+oracle/_ref (oracle/build_ref.py) -- never copied into the repo."""
 import os
 import subprocess
 import sys
@@ -14,10 +14,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _examples_root():
-    for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.isfile(os.path.join(cand, "sf_examples", "train_gym_env.py")):
-            return cand
-    return None
+    ref = os.path.join(ROOT, "oracle", "_ref")
+    return ref if os.path.isfile(os.path.join(ref, "sf_examples", "train_gym_env.py")) else None
 
 
 def _run(args, timeout=600):
@@ -141,7 +139,7 @@ def test_sf_examples_train_gym_env_runs_unmodified(tmp_path):
     script's own docstring (train_gym_env.py:4), the script taken unmodified from the reference, then
     `python -m sf_examples.enjoy_gym_env` on the checkpoint it wrote."""
     if _examples_root() is None:
-        pytest.skip("the reference's sf_examples are not available (baseline/_ref not installed)")
+        pytest.skip("the reference's sf_examples are not available (oracle/_ref not installed)")
     common = ["--algo=APPO", "--use_rnn=False", "--num_envs_per_worker=20", "--policy_workers_per_policy=2", "--recurrence=1",
               "--with_vtrace=False", "--batch_size=512", "--reward_scale=0.1", "--experiment=example_gym_cartpole-v1",
               "--env=CartPole-v1", f"--train_dir={tmp_path}"]
