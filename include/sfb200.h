@@ -27,7 +27,7 @@ extern "C" {
 #pragma GCC visibility push(default) /* everything declared here is exported; the rest of the library is hidden */
 #endif
 
-#define SFB200_ABI_VERSION 1
+#define SFB200_ABI_VERSION 2
 
 /* activation codes (model/model_utils.py:27-35) */
 #define SFB200_ACT_NONE 0
@@ -67,8 +67,8 @@ int sfb200_refresh_tf32_lo(const float* base, void* stream);
  * sfb200_clip_adam_step keeps registered twins current; the transposed copies and the twins after any other write to
  * the weights are refreshed by the refresh_* calls.  sfb200_linear_out_bound derives the bound of a layer's output from
  * the bound of its input: max_n (in_bound * sum_k |W[n][k]| + |b[n]|) (tanh: at most 1); out_bound_dev is FOUR 32-bit words
- * [bound, scratch, counter, -], the middle two zero on entry and on return.  SFB200_TC_F16=0 disables
- * the form (A/B comparison).  No counterpart in the reference (its nn.Linear runs cuBLAS fp32 / CPU). */
+ * [bound, scratch, counter, -], the middle two zero on entry and on return.  No counterpart in the reference (its
+ * nn.Linear runs cuBLAS fp32 / CPU). */
 int sfb200_register_f16_twins(const float* base, void* twins, int64_t n);
 int sfb200_unregister_f16_twins(const float* base);
 int sfb200_refresh_f16_twins(const float* base, void* stream);
@@ -258,16 +258,6 @@ int sfb200_rollout_mlp2_tape(int64_t n_envs, int T, int K1, const float* W1, con
                              int64_t traj_obs_stride, const float* rnn, int rnn_dim, float* traj_rnn_0, int64_t traj_rnn_stride,
                              const double* mean, const double* var, float sub_mean, float inv_scale, float eps, float clip,
                              void* stream);
-/* The whole policy forward of a two-layer MLP (model/encoder.py:72-91 MlpEncoder + actor_critic.py:171-186) up to the head
- * partials in ONE tcgen05 kernel: h1 = act(x W1^T + b1) is produced chunk by chunk in tensor memory and consumed by the
- * layer-2 MMAs without ever reaching shared or global memory; h2 = act(h1 W2^T + b2) is contracted with [Wv ; Wa] in the
- * epilogue (not stored).  Same partial format as sfb200_linear_act_heads_forward -> finish with sfb200_heads_from_partials.
- *   P = sfb200_policy_mlp2_partials(W1, W2, K1, H1, H2, A, engine)   0 -> not covered (needs the 3xTF32 engine, K1 in
- *       {32, 64}, H1 % 32 == 0, H2 % 128 == 0 and <= 512, A <= 8, both weight matrices inside a registered tf32-lo buffer) */
-int sfb200_policy_mlp2_partials(const float* W1, const float* W2, int K1, int H1, int H2, int A, int engine);
-int sfb200_policy_mlp2_heads_forward(const float* x, int64_t ldx, int64_t M, int K1, const float* W1, const float* b1, int H1,
-                                     const float* W2, const float* b2, int H2, int act, int engine, const float* Wv,
-                                     const float* Wa, int A, float* head_partials, void* stream);
 int sfb200_heads_from_partials(const float* head_partials, int P, int64_t rows, int A, const float* bv, const float* ba,
                                float* values, int64_t values_stride, float* logits, int64_t logits_stride,
                                const float* noise, uint64_t philox_seed, uint64_t philox_offset,
@@ -275,22 +265,6 @@ int sfb200_heads_from_partials(const float* head_partials, int P, int64_t rows, 
                                int32_t* env_actions_i32, float* log_prob, int64_t log_prob_stride,
                                const float* policy_version_scalar, float* policy_version_out, int64_t pv_stride,
                                void* stream);
-
-/* The same fused layer, finishing the heads INSIDE the GEMM kernel (no second launch): the n-tile CTAs of every 128-row
- * block count themselves in finish_counters[M/128] (int32, zero before the first call, left at zero); the CTA that arrives
- * last sums the partials of its rows in fixed order and runs the distribution tail.  dist_kind: 0 = Discrete(A),
- * 1 = Tuple of Discretes (num_heads, head_sizes_host), 2 = Box(act_dim) (adaptive_stddev, learned_log_std, tanh_scale;
- * A = 2*act_dim or act_dim).  env_actions: int32 [M] / [M, num_heads], or float32 [M, act_dim] for dist_kind 2.  The other
- * outputs are those of sfb200_heads_forward / _tuple / _continuous. */
-int sfb200_linear_act_heads_forward_fused(
-    const float* x, int64_t ldx, const float* W, const float* b, float* y, int64_t ldy, int64_t M, int N, int K, int act,
-    int engine, const float* Wv, const float* bv, const float* Wa, const float* ba, int A, float* head_partials,
-    int32_t* finish_counters, int dist_kind, int act_dim, int adaptive_stddev, const float* learned_log_std,
-    float tanh_scale, int num_heads, const int32_t* head_sizes_host, float* values, int64_t values_stride, float* logits,
-    int64_t logits_stride, const float* noise, uint64_t philox_seed, uint64_t philox_offset,
-    const int64_t* philox_offset_dev, float* actions_f32, int64_t actions_stride, void* env_actions, float* log_prob,
-    int64_t log_prob_stride, const float* policy_version_scalar, float* policy_version_out, int64_t pv_stride,
-    void* stream);
 
 /* ------------------------------------------------------------- sampler steps ---- */
 /* BatchedVectorEnvRunner.generate_policy_request (algo/sampling/batched_sampling.py:374-388) fused with the

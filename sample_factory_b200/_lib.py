@@ -45,6 +45,14 @@ def parse_header(path: str = HEADER_PATH) -> Dict[str, Tuple[str, List[Tuple[str
     return protos
 
 
+def header_abi_version(path: str = HEADER_PATH) -> int:
+    """SFB200_ABI_VERSION as defined in the header: the version the library built from it must report."""
+    return int(re.search(r"^#define SFB200_ABI_VERSION (\d+)", open(path).read(), flags=re.M).group(1))
+
+
+ABI_VERSION = header_abi_version()
+
+
 def _ctype(t: str):
     if t.endswith("*"):
         return ctypes.c_char_p if t == "const char*" else ctypes.c_void_p
@@ -68,7 +76,7 @@ class _Lib:
             fn = getattr(self.cdll, name)  # AttributeError if the symbol is not exported
             fn.restype = _ctype(ret)
             fn.argtypes = [_ctype(t) for t, _ in args]
-        assert self.cdll.sfb200_abi_version() == 1, "libsfb200 ABI version mismatch"
+        assert self.cdll.sfb200_abi_version() == ABI_VERSION, "libsfb200 ABI version mismatch"
 
     def call(self, name: str, *args):
         """Invoke an `int sfb200_*` entry point; raises SfbError with the library's message on failure."""

@@ -11,17 +11,9 @@ constexpr int SFB_TC_UNSUPPORTED = -1000;   // shape/alignment not handled by th
 int tc_linear_act_forward(const float* x, int64_t ldx, const float* W, const float* b, float* y, int64_t ldy, int64_t M,
                           int N, int K, int act, int engine, cudaStream_t st);
 int tc_linear_heads_partials(int N, int A, int engine);
-struct HeadsFinish;   // heads_tail.cuh
-// fin + fin_counters (both optional): the kernel also finishes the heads (see TcEpilogue::fin_counters in gemm_tc.cu)
 int tc_linear_act_heads_forward(const float* x, int64_t ldx, const float* W, const float* b, float* y, int64_t ldy,
                                 int64_t M, int N, int K, int act, int engine, const float* Wv, const float* Wa, int A,
-                                float* head_part, cudaStream_t st, const HeadsFinish* fin = nullptr,
-                                int* fin_counters = nullptr);
-// fused two-layer policy step (policy_step.cu): number of head partials, or 0 when the model is not covered
-int tc_policy_mlp2_supported(const float* W1, const float* W2, int K1, int H1, int H2, int A, int engine);
-int tc_policy_mlp2_heads_forward(const float* x, int64_t ldx, int64_t M, int K1, const float* W1, const float* b1, int H1,
-                                 const float* W2, const float* b2, int H2, int act, int engine, const float* Wv,
-                                 const float* Wa, int A, float* head_part, cudaStream_t st);
+                                float* head_part, cudaStream_t st);
 // colsum_part (optional, (M/32) * K floats): the dX GEMM's epilogue leaves per-warp column sums of dx there and sets
 // *colsum_fused = 1 when it could (full tiles); the caller then only runs the fixed-order reduce over M/32 partial rows
 int tc_linear_backward(const float* dz, int64_t lddz, const float* x, int64_t ldx, const float* W, int64_t M, int N,

@@ -26,11 +26,13 @@
 
 #include "common.cuh"
 #include "gemm.h"
-#include "heads_tail.cuh"
 #include "tc_ptx.cuh"
 
 namespace sfb {
 
+// Passed to the kernels as a __grid_constant__ parameter: the epilogue reads its fields from the parameter bank where it
+// uses them.  A by-value copy gets promoted into registers for the whole persistent tile loop, which makes the
+// 128-register epilogue warps spill more (ptxas -v).
 struct TcEpilogue {
     int mode;            // 0 plain, 1 act(acc + bias[n]), 2 acc * act'(aux[m,n])
     int act;
@@ -46,11 +48,6 @@ struct TcEpilogue {
     // fused column sums of the OUTPUT (bias gradient of the previous layer = sum over rows of dX): one partial row per
     // (128-row tile, 32-row warp quadrant) -> colsum_part[(m_tile*4 + quadrant)][N]; requires M % 128 == 0, N % 128 == 0
     float* colsum_part;
-    // finish the heads inside this kernel: the n-tile CTAs of a 128-row block count themselves in fin_counters[m_block];
-    // the one that arrives last sums the partials of its rows and runs the distribution tail (sampling, log-prob, ...) --
-    // the separate finishing launch disappears.  fin_counters: M/128 zero-initialised ints, left at zero again.
-    int* fin_counters;
-    HeadsFinish fin;
 };
 
 constexpr int kHeadAP = 9;     // value + up to 8 action outputs
@@ -164,7 +161,6 @@ struct EpiCtx {
     bool vec_ok, aux_vec, bias_vec, st_v8, aux_v8;
     const float* bias_base;
     float out_scale;     // fp16-split engine: 2^-(operand shifts); 1 otherwise
-    bool probe_no_store;
 };
 
 // Epilogue warps 6..13: warp w may touch TMEM lanes [32*(w%4), 32*(w%4)+32); warps 6..9 take columns [0, BN/2) of their
@@ -191,7 +187,6 @@ __device__ __forceinline__ EpiCtx make_epi_ctx(int warp, int lane, const float* 
     ec.bias_vec = epi.bias && (bias_smem || ((reinterpret_cast<uintptr_t>(epi.bias) & 15u) == 0));
     ec.mode = splits == 1 ? epi.mode : 0;
     ec.out_scale = 1.f;
-    ec.probe_no_store = false;
     return ec;
 }
 
@@ -275,13 +270,6 @@ __device__ __forceinline__ void tc_epilogue_tile(uint32_t tmem_slot_addr, uint64
             }
         }
         float* dst = dst_row + c0;
-        if (ec.probe_no_store) {          // SFB200_TA_PROBE=256: how much of a tile is the epilogue's arithmetic + global stores?
-            float t = 0.f;
-#pragma unroll
-            for (int j = 0; j < 32; ++j) t += acc[j];
-            if (t == 123.456f) dst[0] = t;
-            continue;
-        }
         if (fast) {
             // whole row segment in bounds, 128-bit everything; mode / activation resolved once per chunk into
             // a straight-line specialisation (a per-element switch cost 4x the instructions)
@@ -338,7 +326,7 @@ __device__ __forceinline__ void tc_epilogue_tile_heads(uint32_t tmem_slot_addr, 
     float o[CH];
     tmem_drain<BN, CH, SPLIT3, F16>(tmem_slot_addr + ((uint32_t)ec.lane_base << 16) + (uint32_t)ec.col0, o, acc_full_bar, acc_ph,
                                     acc_empty_bar, ec.out_scale);
-    if (m >= M) return;   // (the caller's named barriers come after this function: every thread still reaches them)
+    if (m >= M) return;
     float hp[kHeadAP];
 #pragma unroll
     for (int a = 0; a < kHeadAP; ++a) hp[a] = 0.f;
@@ -388,7 +376,8 @@ __device__ __forceinline__ void tc_epilogue_tile_heads(uint32_t tmem_slot_addr, 
 template <bool A_MN, bool B_MN, int BN, int STAGES, bool SPLIT3>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-               float* __restrict__ C, int64_t ldc, int64_t M, int N, int K, int k_chunk, int splits, TcEpilogue epi) {
+               float* __restrict__ C, int64_t ldc, int64_t M, int N, int K, int k_chunk, int splits,
+               const __grid_constant__ TcEpilogue epi) {
     using S = TcSmem<BN, STAGES>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = smem_align_1024(smem_raw);
@@ -402,7 +391,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     float* bias_s = reinterpret_cast<float*>(smem + STAGES * S::STAGE_BYTES + 512);
 
     constexpr uint32_t ACC_COLS = SPLIT3 ? 2 * BN : BN;   // columns per accumulator slot ([0,BN) main, [BN,2BN) cross)
-    constexpr uint32_t TMEM_COLS = 2 * ACC_COLS;          // two slots: 512 (BN=128, split) .. 128
+    constexpr uint32_t TMEM_COLS = 2 * ACC_COLS;          // two slots: 256 (split) or 128
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tiles_n = (N + BN - 1) / BN;
@@ -604,13 +593,10 @@ template <bool A_MN, bool B_MN, bool SPLIT3, bool HEADS, bool BLO, int TA_OPW, b
 __global__ void __launch_bounds__(ta_threads(TA_OPW), 1)
 gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                   const __grid_constant__ CUtensorMap tmap_b_lo, float* __restrict__ C, int64_t ldc, int64_t M, int N,
-                  int K, int k_chunk, int splits, TcEpilogue epi, int flags, const float* __restrict__ a_bound) {
-    static_assert(!F16 || (!A_MN && !B_MN && SPLIT3 && BLO), "fp16-split engine: K-major operands, weight twins");
+                  int K, int k_chunk, int splits, const __grid_constant__ TcEpilogue epi, const float* __restrict__ a_bound) {
+    static_assert(!F16 || (!A_MN && !B_MN && SPLIT3 && BLO && TA_OPW == 4), "fp16-split engine: K-major operands, weight twins");
     constexpr int BN = 128, STAGES = F16 ? TA_F16_STAGES : TA_STAGES;
     constexpr int KB_K = F16 ? 64 : TBK;                    // k per pipeline stage
-    const int raw_hi = flags & 1;
-    const bool probe_no_b = flags & 2, probe_no_a = flags & 4, probe_no_cross = flags & 8, probe_no_blo = flags & 16;
-    const int a_prefetch = (flags & 32) ? 4 : (flags & 64) ? 8 : (flags & 128) ? 16 : 0;
     constexpr int TA_EPI_WARP0 = 2 + TA_OPW;                // first of the 8 epilogue warps
     using S = TaSmem<STAGES, F16>;
     extern __shared__ uint8_t smem_raw[];
@@ -665,7 +651,7 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                     const int s = it % STAGES;
                     mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
                     uint8_t* sb = smem + s * S::STAGE_BYTES;
-                    mbar_expect_tx(&full[s], ((BLO && !probe_no_blo) ? 2 : 1) * S::B_BYTES + S::A_BYTES);
+                    mbar_expect_tx(&full[s], (BLO ? 2 : 1) * S::B_BYTES + S::A_BYTES);
                     const int k0 = tc.k_begin + kb * KB_K;
                     if (F16) {
                         tma_load_2d(sb + 2 * S::B_BYTES, &tmap_a, &full[s], k0, (int)tc.m0);
@@ -674,10 +660,6 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                         tma_load_2d(sb + S::B_BYTES, &tmap_b_lo, &full[s], k0, tc.n0);    // lo16
                         continue;
                     }
-                    if (!A_MN && a_prefetch && kb + a_prefetch < tc.num_kb)
-                        asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(&tmap_a),
-                                     "r"(k0 + a_prefetch * TBK), "r"((int)tc.m0)
-                                     : "memory");
                     if (A_MN) {
                         for (int j = 0; j < TBM / 32; ++j)
                             tma_load_2d(sb + 2 * S::B_BYTES + j * 4096, &tmap_a, &full[s], (int)tc.m0 + 32 * j, k0);
@@ -691,7 +673,7 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                                 tma_load_2d(sb + S::B_BYTES + j * 4096, &tmap_b_lo, &full[s], tc.n0 + 32 * j, k0);
                     } else {
                         tma_load_2d(sb, &tmap_b, &full[s], k0, tc.n0);
-                        if (BLO && !probe_no_blo) tma_load_2d(sb + S::B_BYTES, &tmap_b_lo, &full[s], k0, tc.n0);
+                        if (BLO) tma_load_2d(sb + S::B_BYTES, &tmap_b_lo, &full[s], k0, tc.n0);
                     }
                 }
             }
@@ -726,7 +708,7 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                         }
                         // [main | cross] (+)= A_hi x [B_hi ; B_lo]   (plain tf32 mode: main (+)= A x B)
                         umma_tf32_ts(tmem_base, a_hi + k * UMMA_K, db_hi + bo, idesc_wide, (kb | k) != 0);
-                        if (SPLIT3 && !probe_no_cross) umma_tf32_ts(tmem_base + BN, a_hi + 32 + k * UMMA_K, db_hi + bo, idesc_cross, 1);
+                        if (SPLIT3) umma_tf32_ts(tmem_base + BN, a_hi + 32 + k * UMMA_K, db_hi + bo, idesc_cross, 1);
                     }
                     umma_commit(&empty[s]);
                     if (kb == nkb - 1) umma_commit(acc_full);
@@ -756,15 +738,12 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                 tc_fence_after();
                 uint8_t* sb = smem + s * S::STAGE_BYTES;
                 if constexpr (F16) {
-                    // 64 k of a tile row = two 128 B swizzled rows (one per 32-k box) -> 32 + 32 packed half2 words of TMEM.
-                    // Four operand warps: a thread converts both boxes of its row; eight: one box each (the warps of a
-                    // lane quadrant work on the same stage at the same time: half the per-stage conversion latency).
-                    constexpr int BOXES = TA_OPW == 8 ? 1 : 2;
-                    const int box0 = TA_OPW == 8 ? ((warp - 2) >> 2) : 0;
-                    uint32_t h16[16 * BOXES], l16[16 * BOXES];
+                    // 64 k of a tile row = two 128 B swizzled rows (one per 32-k box) -> 32 + 32 packed half2 words of TMEM;
+                    // a thread converts both boxes of its row.
+                    uint32_t h16[32], l16[32];
 #pragma unroll
-                    for (int bx = 0; bx < BOXES; ++bx) {
-                        const uint4* arow = reinterpret_cast<const uint4*>(sb + 2 * S::B_BYTES + (box0 + bx) * 16384 + row * 128);
+                    for (int bx = 0; bx < 2; ++bx) {
+                        const uint4* arow = reinterpret_cast<const uint4*>(sb + 2 * S::B_BYTES + bx * 16384 + row * 128);
 #pragma unroll
                         for (int j = 0; j < 8; ++j) {
                             const uint4 q = arow[j ^ sw];
@@ -774,20 +753,18 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                                        l16[bx * 16 + 2 * j + 1]);
                         }
                     }
-                    const uint32_t st_addr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + TA_ACOL0 + (uint32_t)s * 64u +
-                                             (uint32_t)box0 * 16u;
-                    tmem_st_cols<16 * BOXES>(st_addr, h16);
-                    tmem_st_cols<16 * BOXES>(st_addr + 32u, l16);
+                    const uint32_t st_addr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + TA_ACOL0 + (uint32_t)s * 64u;
+                    tmem_st_cols<32>(st_addr, h16);
+                    tmem_st_cols<32>(st_addr + 32u, l16);
                     tmem_st_wait();
                     tc_fence_before();
                     mbar_arrive(&conv[s]);
                     continue;
                 }
+                // hi = the raw fp32 word: the tensor core reads only the top 19 bits of a tf32 operand (truncation), so
+                // only lo has to be formed
                 uint32_t hi[CPT], lo[CPT];
-                if (probe_no_a) {
-#pragma unroll
-                    for (int kk = 0; kk < CPT; ++kk) hi[kk] = lo[kk] = 0u;
-                } else if (A_MN) {
+                if (A_MN) {
                     // MN-major tile: box (row/32) of [32 k][32 rows], k-rows 128 B apart, 32 B chunks XOR (k % 4)
                     // (SWIZZLE_128B_ATOM_32B).  A warp reads one whole 128 B k-row per instruction: conflict-free.
                     const uint8_t* abox = sb + 2 * S::B_BYTES + (row >> 5) * 4096 + (lane & 7) * 4;
@@ -796,13 +773,8 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                     for (int kk = 0; kk < CPT; ++kk) {
                         const int kabs = c0 + kk;
                         const uint32_t v = *reinterpret_cast<const uint32_t*>(abox + kabs * 128 + ((chunk ^ (kabs & 3)) << 5));
-                        if (SPLIT3) {
-                            const uint32_t h = v & 0xffffe000u;
-                            hi[kk] = raw_hi ? v : h;
-                            lo[kk] = __float_as_uint(__uint_as_float(v) - __uint_as_float(h)) & 0xffffe000u;
-                        } else {
-                            hi[kk] = v;
-                        }
+                        hi[kk] = v;
+                        if (SPLIT3) lo[kk] = __float_as_uint(__uint_as_float(v) - __uint_as_float(v & 0xffffe000u)) & 0xffffe000u;
                     }
                 } else {
                     const uint4* arow = reinterpret_cast<const uint4*>(sb + 2 * S::B_BYTES + row * 128);
@@ -812,31 +784,27 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                         const uint32_t v[4] = {q.x, q.y, q.z, q.w};
 #pragma unroll
                         for (int e = 0; e < 4; ++e) {
-                            if (SPLIT3) {
-                                const uint32_t h = v[e] & 0xffffe000u;
-                                hi[4 * j + e] = raw_hi ? v[e] : h;
-                                lo[4 * j + e] = __float_as_uint(__uint_as_float(v[e]) - __uint_as_float(h)) & 0xffffe000u;
-                            } else {
-                                hi[4 * j + e] = v[e];
-                            }
+                            hi[4 * j + e] = v[e];
+                            if (SPLIT3)
+                                lo[4 * j + e] =
+                                    __float_as_uint(__uint_as_float(v[e]) - __uint_as_float(v[e] & 0xffffe000u)) & 0xffffe000u;
                         }
                     }
                 }
                 tmem_st_cols<CPT>(lane_addr + (uint32_t)s * 64u, hi);
                 if (SPLIT3) tmem_st_cols<CPT>(lane_addr + (uint32_t)s * 64u + 32u, lo);
-                if (SPLIT3 && !BLO && !probe_no_b) {
-                    uint4* h4 = reinterpret_cast<uint4*>(sb);
+                if (SPLIT3 && !BLO) {
+                    // B hi stays the raw tile in place (see above); only the lo tile is written
+                    const uint4* h4 = reinterpret_cast<const uint4*>(sb);
                     uint4* l4 = reinterpret_cast<uint4*>(sb + S::B_BYTES);
 #pragma unroll 4
                     for (int i = ct; i < S::B_BYTES / 16; i += NCT) {
                         const uint4 v = h4[i];
-                        uint4 h, l;
-                        h.x = v.x & 0xffffe000u; h.y = v.y & 0xffffe000u; h.z = v.z & 0xffffe000u; h.w = v.w & 0xffffe000u;
-                        l.x = __float_as_uint(__uint_as_float(v.x) - __uint_as_float(h.x)) & 0xffffe000u;
-                        l.y = __float_as_uint(__uint_as_float(v.y) - __uint_as_float(h.y)) & 0xffffe000u;
-                        l.z = __float_as_uint(__uint_as_float(v.z) - __uint_as_float(h.z)) & 0xffffe000u;
-                        l.w = __float_as_uint(__uint_as_float(v.w) - __uint_as_float(h.w)) & 0xffffe000u;
-                        if (!raw_hi) h4[i] = h;     // raw_hi: the tensor core truncates the low 13 mantissa bits itself
+                        uint4 l;
+                        l.x = __float_as_uint(__uint_as_float(v.x) - __uint_as_float(v.x & 0xffffe000u)) & 0xffffe000u;
+                        l.y = __float_as_uint(__uint_as_float(v.y) - __uint_as_float(v.y & 0xffffe000u)) & 0xffffe000u;
+                        l.z = __float_as_uint(__uint_as_float(v.z) - __uint_as_float(v.z & 0xffffe000u)) & 0xffffe000u;
+                        l.w = __float_as_uint(__uint_as_float(v.w) - __uint_as_float(v.w & 0xffffe000u)) & 0xffffe000u;
                         l4[i] = l;
                     }
                 }
@@ -859,7 +827,6 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
         }
         EpiCtx ec = make_epi_ctx<BN, TA_EPI_WARP0>(warp, lane, C, ldc, N, splits, epi, bias_s, S::BIAS_FLOATS);
         if (F16) ec.out_scale = pow2f_int(-(a_shift + kF16WShift));
-        ec.probe_no_store = (flags & 256) != 0;
         uint32_t tile_iter = 0;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++tile_iter) {
             const TileCoord tc = tile_coord(tile, tiles_n, tiles_per_z, BN, K, k_chunk);
@@ -881,25 +848,6 @@ gemm_tc_ta_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                         tc_epilogue_tile_heads<BN, SPLIT3, SFB200_ACT_NONE, F16>(tmem_base, acc_full, tile_iter & 1, acc_empty, tc, ec,
                                                                             C, ldc, M, N, epi, headw_s);
                         break;
-                }
-                if (epi.fin_counters) {
-                    // last-arriving n-tile CTA of this 128-row block finishes the heads (threadFenceReduction pattern)
-                    volatile int* s_last = reinterpret_cast<volatile int*>(tmem_slot + 4);
-                    const int mb = (int)(tc.m0 / TBM);
-                    __threadfence();
-                    asm volatile("bar.sync 1, 256;" ::: "memory");
-                    if (threadIdx.x == TA_EPI_WARP0 * 32) *s_last = (atomicAdd(&epi.fin_counters[mb], 1) == tiles_n - 1) ? 1 : 0;
-                    asm volatile("bar.sync 1, 256;" ::: "memory");
-                    if (*s_last) {
-                        __threadfence();
-                        const float pv = epi.fin.pv_scalar ? *epi.fin.pv_scalar : 0.f;
-                        const uint64_t offset = epi.fin.offset_host + (epi.fin.offset_dev ? (uint64_t)*epi.fin.offset_dev : 0ull);
-                        for (int r = warp - TA_EPI_WARP0; r < TBM; r += 8) {
-                            const int64_t row = tc.m0 + r;
-                            if (row < M) heads_finish_row(epi.head_part, 2 * tiles_n, M, row, lane, epi.fin, pv, offset);
-                        }
-                        if (threadIdx.x == TA_EPI_WARP0 * 32) epi.fin_counters[mb] = 0;
-                    }
                 }
             } else {
                 tc_epilogue_tile<BN, SPLIT3, F16>(tmem_base, acc_full, tile_iter & 1, acc_empty, tc, ec, C, ldc, M, N, splits, epi);
@@ -957,10 +905,11 @@ static bool operand_ok(const float* p, int64_t ld) {
     return ((reinterpret_cast<uintptr_t>(p) & 15u) == 0) && (ld % 4 == 0) && ld > 0;
 }
 
-template <bool A_MN, bool B_MN, int BN, bool SPLIT3>
+// shared-memory-A kernel: N < 128 (every N >= 128 shape runs on the TMEM-A kernel)
+template <bool A_MN, bool B_MN, bool SPLIT3>
 static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, float* C, int64_t ldc, int64_t M, int N, int K,
                      int k_chunk, int splits, const TcEpilogue& epi, cudaStream_t st) {
-    constexpr int STAGES = (BN == 128) ? 3 : 4;
+    constexpr int BN = 64, STAGES = 4;
     using S = TcSmem<BN, STAGES>;
     auto kern = gemm_tc_kernel<A_MN, B_MN, BN, STAGES, SPLIT3>;
     static bool attr_set = false;
@@ -976,18 +925,6 @@ static int launch_tc(const CUtensorMap& ta, const CUtensorMap& tb, float* C, int
     return 0;
 }
 
-// The tensor core reads only the top 19 bits of a tf32 operand (truncation), so the un-masked fp32 value can serve as the
-// "hi" operand and only "lo" has to be written back (measured: bit-identical results, one smem write per element
-// less).  SFB200_TC_RAW_HI=0 restores the explicit mask.
-static bool raw_hi_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TC_RAW_HI");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
 // SFB200_TA_DW_OPW=8 runs the dW-type GEMM (both operands MN-major) with eight operand warps instead of four: 120.8 vs 128.0 us
 // at 32768 x 512 x 512 (tools/dw_bench.py, call r02_y; before the shared-memory address-space fix the two were equal).  Opt-in:
 // the round's GPU budget ended before the full parity suite could be re-run with it as the default.
@@ -996,17 +933,6 @@ static int dw_operand_warps() {
     if (v < 0) {
         const char* e = getenv("SFB200_TA_DW_OPW");
         v = (e && e[0] == '8') ? 8 : 4;
-    }
-    return v;
-}
-
-// SFB200_TA_PROBE (tools/dw_bench.py only; results are garbage): 2 = operand warps skip the B split, 4 = skip the A
-// load / convert, 8 = MMA issuer skips the cross MMA.  Which stage paces the kernel = which skip makes it faster.
-static int ta_probe_bits() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TA_PROBE");
-        v = e ? (atoi(e) & 0x1fe) : 0;   // 16 = skip the B_lo TMA load, 32/64/128 = L2 prefetch of the A tiles 4/8/16 k-blocks ahead
     }
     return v;
 }
@@ -1026,7 +952,7 @@ static int launch_tc_ta_opw(const CUtensorMap& ta, const CUtensorMap& tb, float*
     const int64_t tiles = ceil_div(N, 128) * ceil_div(M, TBM) * splits;
     const int64_t grid = tiles < sm_count() ? tiles : sm_count();
     SFB_CUDA_OK(launch_pdl(kern, dim3((unsigned)grid), dim3(ta_threads(OPW)), (size_t)SMEM, st, ta, tb, tb_lo ? *tb_lo : tb, C, ldc, M,
-                           N, K, k_chunk, splits, epi, (raw_hi_enabled() ? 1 : 0) | ta_probe_bits(), a_bound));
+                           N, K, k_chunk, splits, epi, a_bound));
     SFB_LAUNCH_OK();
     return 0;
 }
@@ -1053,16 +979,6 @@ bool make_tmap_f16(CUtensorMap* out, const uint16_t* base, uint64_t dim0, uint64
     return r == CUDA_SUCCESS;
 }
 
-// SFB200_TC_F16=0 turns the fp16-split engine off (every 3-pass GEMM then runs the tf32 split; A/B comparison)
-static bool f16_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TC_F16");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
 // SFB200_CHECK_F16=1: verify registered fp16 twins against the weights on the device before every use (debugging aid, like
 // SFB200_CHECK_LO for the tf32 twins)
 bool f16_check_enabled() {
@@ -1074,32 +990,14 @@ bool f16_check_enabled() {
     return v == 1;
 }
 
-// SFB200_TC_B_LO=0 ignores registered tf32-lo buffers (A/B comparison)
-static bool blo_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TC_B_LO");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
-// SFB200_TC_A_IN_TMEM=0 selects the shared-memory-A kernel for every shape (A/B comparison, debugging)
-static bool ta_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TC_A_IN_TMEM");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
 // C[M,N] = epi( sum_k A(m,k) B(n,k) ). Returns SFB_TC_UNSUPPORTED when the shape/alignment is not covered.
 static int gemm_tc(bool a_mn, const float* A, int64_t lda, bool b_mn, const float* B, int64_t ldb, float* C, int64_t ldc,
                    int64_t M, int N, int K, int splits, const TcEpilogue& epi, float* ws, bool split3, cudaStream_t st) {
     if (!tc_init()) return SFB_TC_UNSUPPORTED;
     if (!operand_ok(A, lda) || !operand_ok(B, ldb) || M < 1 || N < 8 || K < 8) return SFB_TC_UNSUPPORTED;
     if (M > 0x7fffffff || ceil_div(M, TBM) * ceil_div(N, 64) * 64 > 0x7fffffff) return SFB_TC_UNSUPPORTED;
+    // (A MN-major, B K-major) has no caller and is not instantiated
+    if (a_mn && !b_mn) return SFB_TC_UNSUPPORTED;
     const int BN = (N >= 128) ? 128 : 64;
     CUtensorMap ta, tb;
     bool ok;
@@ -1118,10 +1016,10 @@ static int gemm_tc(bool a_mn, const float* A, int64_t lda, bool b_mn, const floa
     float* out = splits > 1 ? ws : C;
     const int64_t ld_out = splits > 1 ? N : ldc;
 
-    if (epi.head_part && !(BN == 128 && ta_enabled() && !a_mn && !b_mn && splits == 1)) return SFB_TC_UNSUPPORTED;
+    if (epi.head_part && !(BN == 128 && !a_mn && !b_mn && splits == 1)) return SFB_TC_UNSUPPORTED;
     // fp16-split engine: A is a K-major activation buffer with a registered bound, B a weight matrix with registered fp16
     // twins (the transposed twins when B is read MN-major, i.e. dX = dz . W), K a multiple of the 64-k stage
-    if (BN == 128 && ta_enabled() && !a_mn && split3 && splits == 1 && K % 64 == 0 && f16_enabled() && blo_enabled()) {
+    if (BN == 128 && !a_mn && split3 && splits == 1 && K % 64 == 0) {
         const float* a_bound = operand_bound_lookup(A, ((int64_t)(M - 1) * lda + K) * (int64_t)sizeof(float));
         F16Twin tw{nullptr, nullptr};
         if (a_bound) {
@@ -1138,31 +1036,19 @@ static int gemm_tc(bool a_mn, const float* A, int64_t lda, bool b_mn, const floa
             if (!make_tmap_f16(&tb_hi, tw.hi, (uint64_t)K, (uint64_t)N, (uint64_t)K, 64, 128) ||
                 !make_tmap_f16(&tb_lo16, tw.lo, (uint64_t)K, (uint64_t)N, (uint64_t)K, 64, 128))
                 return SFB_TC_UNSUPPORTED;
-            int rc16;
-            static int opw = -1;
-            if (opw < 0) {
-                const char* e = getenv("SFB200_F16_OPW");
-                opw = (e && e[0] == '8') ? 8 : 4;      // (measured: eight operand warps gain nothing, the epilogue spills)
-            }
-            if (epi.head_part) {
-                rc16 = opw == 8 ? launch_tc_ta_opw<false, false, true, true, true, 8, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk,
-                                                                                            splits, epi, st, &tb_lo16, a_bound)
-                                : launch_tc_ta_opw<false, false, true, true, true, 4, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk,
-                                                                                            splits, epi, st, &tb_lo16, a_bound);
-            } else {
-                rc16 = opw == 8 ? launch_tc_ta_opw<false, false, true, false, true, 8, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk,
-                                                                                             splits, epi, st, &tb_lo16, a_bound)
-                                : launch_tc_ta_opw<false, false, true, false, true, 4, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk,
-                                                                                             splits, epi, st, &tb_lo16, a_bound);
-            }
-            return rc16;
+            if (epi.head_part)
+                return launch_tc_ta_opw<false, false, true, true, true, 4, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk, splits,
+                                                                                 epi, st, &tb_lo16, a_bound);
+            return launch_tc_ta_opw<false, false, true, false, true, 4, true>(ta, tb_hi, out, ld_out, M, N, K, k_chunk, splits, epi,
+                                                                              st, &tb_lo16, a_bound);
         }
     }
-    if (BN == 128 && ta_enabled() && (b_mn || !a_mn)) {
-        // A operand from TMEM (gemm_tc_ta_kernel); (A MN-major, B K-major) is not instantiated (no caller)
+    int rc;
+    if (BN == 128) {
+        // A operand from TMEM (gemm_tc_ta_kernel)
         // weight operand with a registered tf32-lo twin (forward layers and dX: B is the weight matrix)
         const int64_t b_extent = b_mn ? (int64_t)(K - 1) * ldb + N : (int64_t)(N - 1) * ldb + K;
-        const float* B_lo = (split3 && !a_mn && raw_hi_enabled() && blo_enabled()) ? tf32_lo_lookup(B, b_extent) : nullptr;
+        const float* B_lo = (split3 && !a_mn) ? tf32_lo_lookup(B, b_extent) : nullptr;
         if (B_lo) {
             CUtensorMap tb_lo;
             bool ok_lo;
@@ -1173,46 +1059,30 @@ static int gemm_tc(bool a_mn, const float* A, int64_t lda, bool b_mn, const floa
                 int rcc = tf32_lo_check(B, B_lo, b_extent, st);
                 if (rcc) return rcc;
             }
-            int rc_lo;
-            if (epi.head_part) rc_lo = launch_tc_ta<false, false, true, true, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
-            else if (!b_mn) rc_lo = launch_tc_ta<false, false, true, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
-            else rc_lo = launch_tc_ta<false, true, true, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
-            if (rc_lo) return rc_lo;
-            if (splits > 1) return splitk_reduce(ws, splits, M, N, C, ldc, st);
-            return 0;
-        }
+            if (epi.head_part) rc = launch_tc_ta<false, false, true, true, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
+            else if (!b_mn) rc = launch_tc_ta<false, false, true, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
+            else rc = launch_tc_ta<false, true, true, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st, &tb_lo);
+        } else {
 #define SFB_TA(AM, BM_)                                                                                                \
     (split3 ? launch_tc_ta<AM, BM_, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st)                     \
             : launch_tc_ta<AM, BM_, false>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st))
-        int rc_ta;
-        if (epi.head_part) {
-            rc_ta = split3 ? launch_tc_ta<false, false, true, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st)
-                           : launch_tc_ta<false, false, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st);
-        } else if (!a_mn && !b_mn) rc_ta = SFB_TA(false, false);
-        else if (!a_mn && b_mn) rc_ta = SFB_TA(false, true);
-        else rc_ta = SFB_TA(true, true);
+            if (epi.head_part) {
+                rc = split3 ? launch_tc_ta<false, false, true, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st)
+                            : launch_tc_ta<false, false, false, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st);
+            } else if (!a_mn && !b_mn) rc = SFB_TA(false, false);
+            else if (!a_mn && b_mn) rc = SFB_TA(false, true);
+            else rc = SFB_TA(true, true);
 #undef SFB_TA
-        if (rc_ta) return rc_ta;
-        if (splits > 1) return splitk_reduce(ws, splits, M, N, C, ldc, st);
-        return 0;
-    }
-
-#define SFB_TC(AM, BM_, BNv)                                                                                           \
-    (split3 ? launch_tc<AM, BM_, BNv, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st)                   \
-            : launch_tc<AM, BM_, BNv, false>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st))
-    int rc;
-    if (BN == 128) {
-        if (!a_mn && !b_mn) rc = SFB_TC(false, false, 128);
-        else if (!a_mn && b_mn) rc = SFB_TC(false, true, 128);
-        else if (a_mn && b_mn) rc = SFB_TC(true, true, 128);
-        else return SFB_TC_UNSUPPORTED;
+        }
     } else {
-        if (!a_mn && !b_mn) rc = SFB_TC(false, false, 64);
-        else if (!a_mn && b_mn) rc = SFB_TC(false, true, 64);
-        else if (a_mn && b_mn) rc = SFB_TC(true, true, 64);
-        else return SFB_TC_UNSUPPORTED;
-    }
+#define SFB_TC(AM, BM_)                                                                                                \
+    (split3 ? launch_tc<AM, BM_, true>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st)                         \
+            : launch_tc<AM, BM_, false>(ta, tb, out, ld_out, M, N, K, k_chunk, splits, epi, st))
+        if (!a_mn && !b_mn) rc = SFB_TC(false, false);
+        else if (!a_mn && b_mn) rc = SFB_TC(false, true);
+        else rc = SFB_TC(true, true);
 #undef SFB_TC
+    }
     if (rc) return rc;
     if (splits > 1) return splitk_reduce(ws, splits, M, N, C, ldc, st);
     return 0;
@@ -1227,22 +1097,18 @@ int tc_linear_act_forward(const float* x, int64_t ldx, const float* W, const flo
 // Number of head partials the fused forward produces per row for an N-wide layer, or 0 when the fused path does not
 // cover the shape (callers then run the layer and the heads kernel separately).
 int tc_linear_heads_partials(int N, int A, int engine) {
-    if (engine == SFB200_GEMM_SIMT_FP32 || !tc_init() || !ta_enabled()) return 0;
+    if (engine == SFB200_GEMM_SIMT_FP32 || !tc_init()) return 0;
     if (N % 128 != 0 || N > 512 || A < 1 || A + 1 > kHeadAP) return 0;
     return 2 * (N / 128);
 }
 
 int tc_linear_act_heads_forward(const float* x, int64_t ldx, const float* W, const float* b, float* y, int64_t ldy,
                                 int64_t M, int N, int K, int act, int engine, const float* Wv, const float* Wa, int A,
-                                float* head_part, cudaStream_t st, const HeadsFinish* fin, int* fin_counters) {
+                                float* head_part, cudaStream_t st) {
     if (tc_linear_heads_partials(N, A, engine) == 0 || !b) return SFB_TC_UNSUPPORTED;
     if (y && (ldy % 4 != 0 || (reinterpret_cast<uintptr_t>(y) & 15u))) return SFB_TC_UNSUPPORTED;
     if (reinterpret_cast<uintptr_t>(head_part) & 15u) return SFB_TC_UNSUPPORTED;
     TcEpilogue epi{1, act, b, nullptr, 0, Wv, Wa, A, head_part};
-    if (fin && fin_counters) {
-        epi.fin = *fin;
-        epi.fin_counters = fin_counters;
-    }
     return gemm_tc(false, x, ldx, false, W, K, y, y ? ldy : N, M, N, K, 1, epi, nullptr, engine == SFB200_GEMM_TC_3XTF32, st);
 }
 
@@ -1259,7 +1125,7 @@ int tc_linear_backward(const float* dz, int64_t lddz, const float* x, int64_t ld
         // dx[m,k] = (sum_n dz[m,n] W[n,k]) * act_prev'(x[m,k]): A = dz K-major, B(k, n) = W[n,k] MN-major
         TcEpilogue e{act_prev == SFB200_ACT_NONE ? 0 : 2, act_prev, nullptr, x, ldx};
         // db_prev = column sums of dx, folded into this GEMM's epilogue when every tile is full (TMEM-A kernel, BN = 128)
-        const bool fuse_cs = colsum_part && M % 128 == 0 && K % 128 == 0 && ta_enabled() && lddx % 4 == 0 &&
+        const bool fuse_cs = colsum_part && M % 128 == 0 && K % 128 == 0 && lddx % 4 == 0 &&
                              (act_prev == SFB200_ACT_NONE || (ldx % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15u) == 0)) &&
                              (reinterpret_cast<uintptr_t>(dx) & 15u) == 0;
         if (fuse_cs) e.colsum_part = colsum_part;

@@ -831,42 +831,6 @@ int sfb200_heads_from_partials_tuple(const float* head_partials, int P, int64_t 
                                     philox_offset_dev, policy_version_scalar, (cudaStream_t)stream);
 }
 
-int sfb200_linear_act_heads_forward_fused(
-    const float* x, int64_t ldx, const float* W, const float* b, float* y, int64_t ldy, int64_t M, int N, int K, int act,
-    int engine, const float* Wv, const float* bv, const float* Wa, const float* ba, int A, float* head_partials,
-    int32_t* finish_counters, int dist_kind, int act_dim, int adaptive_stddev, const float* learned_log_std,
-    float tanh_scale, int num_heads, const int32_t* head_sizes_host, float* values, int64_t values_stride, float* logits,
-    int64_t logits_stride, const float* noise, uint64_t philox_seed, uint64_t philox_offset,
-    const int64_t* philox_offset_dev, float* actions_f32, int64_t actions_stride, void* env_actions, float* log_prob,
-    int64_t log_prob_stride, const float* policy_version_scalar, float* policy_version_out, int64_t pv_stride,
-    void* stream) {
-    SFB_CHECK_ARG(x && W && b && Wv && bv && Wa && ba && head_partials && finish_counters && values && M >= 0 && N > 0 && K > 0,
-                  "linear_act_heads_forward_fused: bad arguments");
-    SFB_CHECK_ARG(dist_kind >= 0 && dist_kind <= 2, "linear_act_heads_forward_fused: dist_kind 0 categorical, 1 tuple, 2 Gaussian");
-    if (M == 0) return 0;
-    HeadsOut out{values, values_stride, logits, logits_stride, actions_f32, actions_stride, nullptr, log_prob,
-                 log_prob_stride, policy_version_out, pv_stride, 0, 0, nullptr, 0.f, nullptr};
-    if (dist_kind == 2) {
-        if (int rc = make_gaussian_out(out, act_dim, adaptive_stddev, learned_log_std, tanh_scale, values, values_stride, logits,
-                                       logits_stride, actions_f32, actions_stride, (float*)env_actions, log_prob,
-                                       log_prob_stride, policy_version_out, pv_stride))
-            return rc;
-        SFB_CHECK_ARG(A == (adaptive_stddev ? 2 * act_dim : act_dim), "linear_act_heads_forward_fused: A does not match act_dim");
-    } else {
-        out.env_actions = (int32_t*)env_actions;
-        if (dist_kind == 1)
-            if (int rc = make_tuple_out(out, A, num_heads, head_sizes_host)) return rc;
-    }
-    if (int rc = apply_sampling_mode(out, A)) return rc;
-    const HeadsFinish fin{out, bv, ba, noise, philox_seed, philox_offset, philox_offset_dev, policy_version_scalar, A};
-    int rc = tc_linear_act_heads_forward(x, ldx, W, b, y, ldy, M, N, K, act, engine, Wv, Wa, A, head_partials,
-                                         (cudaStream_t)stream, &fin, finish_counters);
-    SFB_CHECK_ARG(rc != SFB_TC_UNSUPPORTED,
-                  "linear_act_heads_forward_fused: shape/engine not covered (N=%d K=%d A=%d engine=%d); "
-                  "sfb200_linear_heads_partials() tells when to use the separate calls", N, K, A, engine);
-    return rc;
-}
-
 int sfb200_heads_forward_continuous(const float* h, int64_t ldh, int64_t rows, int H, int act_dim, int adaptive_stddev,
                                     const float* Wv, const float* bv, const float* Wa, const float* ba,
                                     const float* learned_log_std, float tanh_scale, float* values,
@@ -922,8 +886,7 @@ int sfb200_heads_backward(const float* h, int64_t ldh, int64_t rows, int H, int 
     const bool vec2 = vec_common && (H % 2 == 0) && (H / 2 <= 256) && (256 % (H / 2) == 0) && rows >= 16384;
     const bool vec4 = vec_common && (H % 4 == 0) && (H / 4 <= 256) && (256 % (H / 4) == 0);
     // pipelined row loads (see heads_backward_pipe_kernel): rows per thread and tile must be a multiple of the queue depth
-    static const int hb_pipe = [] { const char* e = getenv("SFB200_HB_PIPE"); return e ? atoi(e) : 1; }();
-    const bool pipe = vec2 && hb_pipe && (kHbTile / (256 / (H / 2))) % 8 == 0;
+    const bool pipe = vec2 && (kHbTile / (256 / (H / 2))) % 8 == 0;
     int64_t groups = (int64_t)sm_count() * (pipe ? 3 : (vec2 ? 4 : 2));
     if (groups > kHeadsMaxGroups) groups = kHeadsMaxGroups;
     int64_t rpg = ceil_div(rows, groups);

@@ -1,5 +1,5 @@
-// Row tails of the policy/value heads, shared by heads.cu (stand-alone kernels) and gemm_tc.cu (the fused GEMM finishes the
-// heads in its last-arriving CTA): lane a of a warp holds output a of one row (0 = value, 1.. = distribution_linear rows).
+// Row tails of the policy/value heads, shared by heads.cu (stand-alone kernels, sampler step tail) and rollout_fused.cu (the
+// persistent rollout kernel): lane a of a warp holds output a of one row (0 = value, 1.. = distribution_linear rows).
 #pragma once
 #include <curand_kernel.h>
 

@@ -90,7 +90,7 @@ __device__ __forceinline__ uint32_t cluster_ctarank() {
     return r;
 }
 
-// bounded spin (same as policy_step.cu): a protocol bug traps instead of hanging the GPU
+// bounded spin: a protocol bug traps instead of hanging the GPU
 __device__ __forceinline__ void rf_wait(uint64_t* bar, uint32_t parity) {
     uint32_t done = 0;
     uint64_t t0 = 0;
@@ -585,20 +585,11 @@ int tc_rollout_mlp2_supported(const float* W1, const float* W2, int K1, int H1, 
 }
 
 // fp16-split form (common.cuh): taken when the weights have registered fp16 twins and both activation buffers (x_norm, the
-// h1 scratch) have registered bounds; SFB200_TC_F16=0 keeps the tf32 split
-static bool rollout_f16_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("SFB200_TC_F16");
-        v = (e && e[0] == '0') ? 0 : 1;
-    }
-    return v == 1;
-}
-
+// h1 scratch) have registered bounds
 int tc_rollout_mlp2_tape(const float* W1, const float* W2, int act, int engine, const RolloutArgs& a_in, cudaStream_t st) {
     if (!tc_rollout_mlp2_supported(W1, W2, a_in.K1, a_in.H1, a_in.H2, a_in.A, engine)) return SFB_TC_UNSUPPORTED;
     RolloutArgs a = a_in;
-    if (rollout_f16_enabled() && a.K1 % 64 == 0 && a.H1 % 64 == 0) {
+    if (a.K1 % 64 == 0 && a.H1 % 64 == 0) {
         const F16Twin t1 = f16_twin_lookup(W1, (int64_t)a.H1 * a.K1), t2 = f16_twin_lookup(W2, (int64_t)a.H2 * a.H1);
         const float* bx = operand_bound_lookup(a.x_norm, a.N * a.K1 * (int64_t)sizeof(float));
         const float* bh = operand_bound_lookup(a.h1, a.N * a.H1 * (int64_t)sizeof(float));

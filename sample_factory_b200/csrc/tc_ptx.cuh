@@ -1,5 +1,5 @@
 // tcgen05 / TMA / mbarrier PTX wrappers, UMMA descriptors and compile-time activations shared by the GEMM engine
-// (gemm_tc.cu) and the fused policy-step kernel (policy_step.cu).  sm_100a only.
+// (gemm_tc.cu) and the persistent rollout kernel (rollout_fused.cu).  sm_100a only.
 #pragma once
 #include <cuda.h>
 #include <cudaTypedefs.h>

@@ -394,49 +394,26 @@ def linear_act_heads_forward_fused(x: Tensor, W: Tensor, b: Tensor, out: Optiona
                                    head_sizes=None, act_dim: int = 0, adaptive_stddev: bool = True,
                                    learned_log_std: Optional[Tensor] = None, tanh_scale: float = 0.0,
                                    continuous: bool = False) -> None:
-    """Last hidden layer + heads + distribution tail in ONE launch (the last-arriving n-tile CTA of every 128-row block
-    finishes the heads).  finish_counters: int32 [ceil(M/128)] zeros, owned by the caller."""
-    M, K = x.shape
-    N = W.shape[0]
-    A = Wa.shape[0]
-    assert W.shape[1] == K and W.is_contiguous() and Wa.is_contiguous() and Wv.is_contiguous()
-    assert out is None or out.shape == (M, N)
-    P = linear_heads_partials(N, A, engine)
-    assert P > 0 and head_partials.numel() >= P * M * HEAD_PART_PAD and head_partials.is_contiguous()
-    assert finish_counters.dtype == I32 and finish_counters.numel() * 128 >= M
-    assert noise is None or noise.is_contiguous()
-    kind = 2 if continuous else (1 if head_sizes else 0)
-    env_ptr = None if env_actions is None else _p(env_actions, F32 if continuous else I32)
-    lib().call("sfb200_linear_act_heads_forward_fused", _p(x, F32), x.stride(0), _p(W, F32), _p(b, F32), _p(out, F32),
-               0 if out is None else out.stride(0), M, N, K, act, engine, _p(Wv, F32), _p(bv, F32), _p(Wa, F32), _p(ba, F32),
-               A, _p(head_partials, F32), _p(finish_counters, I32), kind, act_dim, int(adaptive_stddev),
-               _p(learned_log_std, F32), float(tanh_scale), len(head_sizes) if head_sizes else 0,
-               _seg_array(head_sizes) if head_sizes else None, values.data_ptr(), values_stride,
-               None if logits is None else logits.data_ptr(), logits_stride, _p(noise, F32), philox_seed, philox_offset,
-               _p(philox_offset_dev, I64), None if actions_f32 is None else actions_f32.data_ptr(), actions_stride, env_ptr,
-               None if log_prob is None else log_prob.data_ptr(), log_prob_stride, _p(policy_version_scalar, F32),
-               None if policy_version_out is None else policy_version_out.data_ptr(), pv_stride, _stream())
-
-
-def policy_mlp2_partials(W1: Tensor, W2: Tensor, A: int, engine: int) -> int:
-    """head partials per row the fused two-layer policy step produces, 0 when the model is not covered"""
-    H1, K1 = W1.shape
-    H2 = W2.shape[0]
-    if W2.shape[1] != H1 or not (W1.is_contiguous() and W2.is_contiguous()):
-        return 0
-    return lib().query("sfb200_policy_mlp2_partials", _p(W1, F32), _p(W2, F32), K1, H1, H2, A, engine)
-
-
-def policy_mlp2_heads_forward(x: Tensor, W1: Tensor, b1: Tensor, W2: Tensor, b2: Tensor, act: int, engine: int, Wv: Tensor,
-                              Wa: Tensor, head_partials: Tensor) -> None:
-    """x [M, K1] -> partial head dot products of act(act(x W1^T + b1) W2^T + b2) (one tcgen05 kernel, csrc/policy_step.cu)"""
-    M, K1 = x.shape
-    H1, H2, A = W1.shape[0], W2.shape[0], Wa.shape[0]
-    assert Wv.is_contiguous() and Wa.is_contiguous() and Wv.numel() == H2 and Wa.shape[1] == H2
-    P = 4 * (H2 // 128)
-    assert head_partials.numel() >= P * M * HEAD_PART_PAD
-    lib().call("sfb200_policy_mlp2_heads_forward", _p(x, F32), x.stride(0), M, K1, _p(W1, F32), _p(b1, F32), H1, _p(W2, F32),
-               _p(b2, F32), H2, act, engine, _p(Wv, F32), _p(Wa, F32), A, _p(head_partials, F32), _stream())
+    """Last hidden layer + heads + distribution tail: linear_act_heads_forward, then the matching
+    heads_from_partials{,_tuple,_continuous}.  This once was one launch that finished the heads inside the GEMM; that
+    kernel measured slower (profiles/r01_l_heads_finish_in_gemm.md) and was removed.  `finish_counters` is no longer
+    used (left untouched).  The function keeps its name and signature because existing callers look it up by name
+    (bench.py times it alongside linear_act_heads_forward)."""
+    linear_act_heads_forward(x, W, b, out, act, engine, Wv, Wa, head_partials)
+    P = linear_heads_partials(W.shape[0], Wa.shape[0], engine)
+    kw = dict(logits=logits, logits_stride=logits_stride, noise=noise, philox_seed=philox_seed, philox_offset=philox_offset,
+              philox_offset_dev=philox_offset_dev, actions_f32=actions_f32, actions_stride=actions_stride,
+              env_actions=env_actions, log_prob=log_prob, log_prob_stride=log_prob_stride,
+              policy_version_scalar=policy_version_scalar, policy_version_out=policy_version_out, pv_stride=pv_stride)
+    M = x.shape[0]
+    if continuous:
+        heads_from_partials_continuous(head_partials, P, M, bv, ba, act_dim=act_dim, adaptive_stddev=adaptive_stddev,
+                                       learned_log_std=learned_log_std, tanh_scale=tanh_scale, values=values,
+                                       values_stride=values_stride, **kw)
+    elif head_sizes:
+        heads_from_partials_tuple(head_partials, P, M, bv, ba, head_sizes, values=values, values_stride=values_stride, **kw)
+    else:
+        heads_from_partials(head_partials, P, M, bv, ba, values=values, values_stride=values_stride, **kw)
 
 
 def heads_from_partials(head_partials: Tensor, P: int, rows: int, bv: Tensor, ba: Tensor, values: Tensor,

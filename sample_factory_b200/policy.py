@@ -9,7 +9,6 @@ activated layer output is stored only if the caller needs it (the learner's back
 """
 from __future__ import annotations
 
-import os
 from typing import Callable, Dict, List, Optional
 
 import torch
@@ -54,27 +53,6 @@ class HeadsPlan:
             self.P = ops.linear_heads_partials(spec.tail_input_size, spec.num_linear_action_outputs, engine)
         if self.P > 0:
             self.part = torch.empty(self.P * max_rows * ops.HEAD_PART_PAD, dtype=torch.float32, device=model.device)
-            # optional: the GEMM finishes the heads itself (last-arriving CTA per 128-row block; these are its arrival
-            # counters).  Measured on B200 (profiles/r01_l_heads_finish_in_gemm.md): one launch less per policy step but
-            # the finishing CTA walks its 128 rows 16 deep per warp -> +25 us per step (28.0M vs 37.3M env-steps/s), so
-            # the separate, fully parallel heads_from_partials launch stays the default.
-            self.counters = torch.zeros((max_rows + 127) // 128, dtype=torch.int32, device=model.device)
-            self.finish_in_gemm = os.environ.get("SFB200_HEADS_FINISH_IN_GEMM", "0") == "1"
-        # two-layer MLP policies (BASELINE cfg-2): both layers + the head partials in ONE tcgen05 kernel whenever the last
-        # hidden activation is not needed afterwards (sampler policy step, learner bootstrap value) -- csrc/policy_step.cu.
-        # Opt-in (SFB200_POLICY_FUSED=1): measured on B200 (profiles/r02_e_*) the fused kernel is faster cold (33.5 vs
-        # 25.2 + 15.6 us under ncu) but slower inside the replayed rollout (29.2 vs 26.5 us warm: it re-computes layer 1 in each
-        # of the four column CTAs, +50 % MMA work, and the tf32 MMA rate is what bounds both), so the per-layer launches stay
-        # the default.
-        self.mlp2 = False
-        self.P_mlp2 = 0
-        if (self.P > 0 and self.conv is None and not spec.use_rnn and not spec.decoder_mlp_layers and
-                len(spec.fc_encoder_layers) == 2 and os.environ.get("SFB200_POLICY_FUSED", "0") == "1"):
-            (W1, _), (W2, _) = model.encoder_layers()
-            self.P_mlp2 = ops.policy_mlp2_partials(W1, W2, spec.num_linear_action_outputs, engine)
-            self.mlp2 = self.P_mlp2 > 0
-            if self.P_mlp2 > self.P:     # (32-column partial groups: twice as many partials as the per-layer epilogue leaves)
-                self.part = torch.empty(self.P_mlp2 * max_rows * ops.HEAD_PART_PAD, dtype=torch.float32, device=model.device)
 
 
 def forward_policy(model: PolicyModel, x: Tensor, outs: List[Tensor], act: int, engine: int, plan: HeadsPlan,
@@ -93,14 +71,6 @@ def forward_policy(model: PolicyModel, x: Tensor, outs: List[Tensor], act: int, 
     Wa, ba = model.actor
     n_mlp = len(enc) + len(dec)
     fused = plan.P > 0
-    if plan.mlp2 and not store_tail and not plan.finish_in_gemm:
-        (W1, b1), (W2, b2) = enc
-        ops.policy_mlp2_heads_forward(x, W1, b1, W2, b2, act, engine, Wv, Wa, plan.part)
-        if finish_fn is not None:
-            finish_fn(plan.part, plan.P_mlp2, M, bv, ba)
-        else:
-            _heads(model, None, Wv, bv, Wa, ba, True, plan, M, heads_kwargs, P=plan.P_mlp2)
-        return None
     k = 0
     tail: Optional[Tensor] = x
     for group, layers in (("enc", enc), ("dec", dec)):
@@ -108,14 +78,6 @@ def forward_policy(model: PolicyModel, x: Tensor, outs: List[Tensor], act: int, 
             tail = rnn_fn(tail)
         for (W, b) in layers:
             last = fused and k == n_mlp - 1
-            if last and plan.finish_in_gemm:
-                out = outs[k][:M] if store_tail else None
-                sp = model.spec
-                dk = model.dist_kwargs() if sp.continuous else {}
-                ops.linear_act_heads_forward_fused(tail, W, b, out, act, engine, Wv, bv, Wa, ba, plan.part, plan.counters,
-                                                   **heads_kwargs, head_sizes=sp.action_segments, continuous=sp.continuous,
-                                                   **dk)
-                return out
             if last:
                 out = outs[k][:M] if store_tail else None
                 ops.linear_act_heads_forward(tail, W, b, out, act, engine, Wv, Wa, plan.part)
@@ -152,20 +114,19 @@ def _forward_separate(model: PolicyModel, x: Tensor, act: int, engine: int, plan
 
 
 def _heads(model: PolicyModel, tail: Tensor, Wv: Tensor, bv: Tensor, Wa: Tensor, ba: Tensor, fused: bool, plan: HeadsPlan,
-           M: int, heads_kwargs: Dict, P: Optional[int] = None) -> None:
-    P = plan.P if P is None else P
+           M: int, heads_kwargs: Dict) -> None:
     if model.spec.continuous:   # Box action space: Gaussian heads (action_distributions.py:290-323)
         dk = model.dist_kwargs()
         if fused:
-            ops.heads_from_partials_continuous(plan.part, P, M, bv, ba, **dk, **heads_kwargs)
+            ops.heads_from_partials_continuous(plan.part, plan.P, M, bv, ba, **dk, **heads_kwargs)
         else:
             ops.heads_forward_continuous(tail, Wv, bv, Wa, ba, **dk, **heads_kwargs)
     elif model.spec.action_segments:   # Tuple of Discretes: independent categorical heads (action_distributions.py:197-286)
         if fused:
-            ops.heads_from_partials_tuple(plan.part, P, M, bv, ba, model.spec.action_segments, **heads_kwargs)
+            ops.heads_from_partials_tuple(plan.part, plan.P, M, bv, ba, model.spec.action_segments, **heads_kwargs)
         else:
             ops.heads_forward_tuple(tail, Wv, bv, Wa, ba, model.spec.action_segments, **heads_kwargs)
     elif fused:
-        ops.heads_from_partials(plan.part, P, M, bv, ba, **heads_kwargs)
+        ops.heads_from_partials(plan.part, plan.P, M, bv, ba, **heads_kwargs)
     else:
         ops.heads_forward(tail, Wv, bv, Wa, ba, **heads_kwargs)

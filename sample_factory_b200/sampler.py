@@ -100,16 +100,16 @@ class DeviceSampler:
         self._eager_rollouts = 0
         self.kernel_launches_per_rollout = 0
         # Fused step tail (csrc/heads.cu sampler_tail_tape_kernel): for the synthetic tape env the heads' finishing step,
-        # the env step, post-step(t) and pre-step(t+1) are ONE launch -- with the fused two-layer policy kernel a policy
-        # step is two launches.  Needs the fused-partials heads path, a plain Discrete action space, float32 observations,
-        # no recurrent core and an env whose step is the tape rule.  SFB200_TAIL_FUSED=0 restores the separate launches.
+        # the env step, post-step(t) and pre-step(t+1) are ONE launch.  Needs the fused-partials heads path, a plain Discrete
+        # action space, float32 observations, no recurrent core and an env whose step is the tape rule.  SFB200_TAIL_FUSED=0
+        # restores the separate launches.
         import os
 
         from .envs import TapeVecEnv
         self.fused_tail = (os.environ.get("SFB200_TAIL_FUSED", "1") != "0" and type(env) is TapeVecEnv and
                            not env.continuous and not env.action_segments and not env.with_action_mask and
                            not env.obs_uint8 and self.rnn is None and self.heads_plan.P > 0 and
-                           not self.heads_plan.finish_in_gemm and not self.heads_plan.separate and
+                           not self.heads_plan.separate and
                            not spec.continuous and not spec.action_segments)
         # Whole rollout as ONE persistent kernel (csrc/rollout_fused.cu): clusters of H2/128 CTAs own a 128-env row block for
         # all T steps.  Same conditions as the fused tail plus a two-layer MLP the kernel covers.  SFB200_ROLLOUT_FUSED=0

@@ -1355,81 +1355,3 @@ def test_heads_forward_tuple(dev):
     assert (logits.cpu() - logits_ref).abs().max().item() < TOL
     assert torch.equal(actions.cpu().long(), a_ref) and torch.equal(env_actions.cpu().long(), a_ref)
     assert (lp.cpu() - lp_ref).abs().max().item() < 2 * TOL
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("M,K1,H1,H2,A,act", [(4096, 64, 512, 512, 8, "elu"), (300, 64, 512, 512, 8, "elu"),
-                                              (1000, 32, 256, 128, 3, "relu"), (129, 64, 96, 256, 5, "tanh"),
-                                              (2048, 64, 1024, 384, 8, "elu")])
-def test_policy_mlp2_heads_forward(dev, M, K1, H1, H2, A, act):
-    """sfb200_policy_mlp2_heads_forward (both MLP layers + head partials in one tcgen05 kernel, h1 only ever in tensor
-    memory) == the per-layer path (sfb200_linear_act_forward + sfb200_linear_act_heads_forward) on the same weights, and
-    == a float64 torch reference at fp32-parity tolerance; action indices identical."""
-    ops = _ops()
-    if not ops.tc_available():
-        pytest.skip("tcgen05 engine not available")
-    engine = ops.GEMM_TC_3XTF32
-    flat = torch.empty(H1 * K1 + H2 * H1, device=dev)
-    lo = torch.empty_like(flat)
-    flat[: H1 * K1] = (torch.randn(H1, K1, generator=g(70)) / math.sqrt(K1)).reshape(-1).to(dev)
-    flat[H1 * K1:] = (torch.randn(H2, H1, generator=g(71)) / math.sqrt(H1)).reshape(-1).to(dev)
-    ops.register_tf32_lo(flat, lo)
-    try:
-        ops.refresh_tf32_lo(flat)
-        W1, W2 = flat[: H1 * K1].view(H1, K1), flat[H1 * K1:].view(H2, H1)
-        b1 = (torch.randn(H1, generator=g(72)) * 0.1).to(dev)
-        b2 = (torch.randn(H2, generator=g(73)) * 0.1).to(dev)
-        Wv = (torch.randn(1, H2, generator=g(74)) / math.sqrt(H2)).to(dev)
-        Wa = (torch.randn(A, H2, generator=g(75)) / math.sqrt(H2)).to(dev)
-        bv = torch.randn(1, generator=g(76)).to(dev)
-        ba = (torch.randn(A, generator=g(77)) * 0.1).to(dev)
-        # strided rows (the learner's bootstrap forward reads obs[:, T] in place)
-        xbuf = torch.randn(M, 3 * K1, generator=g(78)).to(dev)
-        x = xbuf[:, K1: 2 * K1]
-        noise = torch.empty(M, A).exponential_(generator=g(79)).to(dev)
-        P = ops.policy_mlp2_partials(W1, W2, A, engine)
-        assert P == 4 * (H2 // 128)
-        actc = ops.ACT[act]
-        pvs = torch.full((1,), 3.0, device=dev)
-
-        def outs():
-            return dict(values=torch.empty(M, device=dev), logits=torch.empty(M, A, device=dev),
-                        actions=torch.empty(M, device=dev), env_actions=torch.empty(M, dtype=torch.int32, device=dev),
-                        lp=torch.empty(M, device=dev), pv=torch.empty(M, device=dev))
-
-        def kw(o):
-            return dict(values=o["values"], values_stride=1, logits=o["logits"], logits_stride=A, noise=noise,
-                        actions_f32=o["actions"], actions_stride=1, env_actions=o["env_actions"], log_prob=o["lp"],
-                        log_prob_stride=1, policy_version_scalar=pvs, policy_version_out=o["pv"], pv_stride=1)
-
-        part = torch.full((P * M * ops.HEAD_PART_PAD,), float("nan"), device=dev)
-        o_f = outs()
-        ops.policy_mlp2_heads_forward(x, W1, b1, W2, b2, actc, engine, Wv, Wa, part)
-        ops.heads_from_partials(part, P, M, bv, ba, **kw(o_f))
-        # per-layer path
-        h1 = torch.empty(M, H1, device=dev)
-        part2 = torch.full_like(part, float("nan"))
-        o_s = outs()
-        ops.linear_act_forward(x, W1, b1, h1, actc, engine)
-        P2 = ops.linear_heads_partials(H2, A, engine)
-        if P2 > 0:
-            ops.linear_act_heads_forward(h1, W2, b2, None, actc, engine, Wv, Wa, part2)
-            ops.heads_from_partials(part2, P2, M, bv, ba, **kw(o_s))
-            for k in ("values", "logits", "lp"):
-                assert torch.allclose(o_f[k], o_s[k], rtol=0, atol=2e-6), (k, float((o_f[k] - o_s[k]).abs().max()))
-            assert torch.equal(o_f["env_actions"], o_s["env_actions"])
-        # float64 reference
-        fn = {"elu": torch.nn.functional.elu, "relu": torch.relu, "tanh": torch.tanh}[act]
-        xd = x.double()
-        r1 = fn(xd @ W1.double().t() + b1.double())
-        r2 = fn(r1 @ W2.double().t() + b2.double())
-        v_ref = (r2 @ Wv.double().t()).view(-1) + bv.double()
-        l_ref = r2 @ Wa.double().t() + ba.double()
-        assert float((o_f["values"].double() - v_ref).abs().max()) < 1e-5
-        assert float((o_f["logits"].double() - l_ref).abs().max()) < 1e-5
-        p = torch.softmax(l_ref, -1)
-        a_ref = torch.argmax(p / noise.double(), -1).to(torch.int32)
-        assert float((o_f["env_actions"] != a_ref).float().mean()) < 2e-3     # (only near-ties may flip at 1e-6)
-        assert torch.all(o_f["pv"] == 3.0)
-    finally:
-        ops.unregister_tf32_lo(flat)
